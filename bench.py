@@ -4,6 +4,7 @@ Gvoxel/s on 1024x1024 rectified tiles, disp_range 128, census 5x5 + 8-path MGM, 
 
     python bench.py --gpus N --steps K --warmup W              # our CUDA engine
     python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU `mgm` on host cores
+    python bench.py --steps K --dump-outputs DIR               # + the last timed step's outputs as DIR/*.npy, to compare builds
 
 A "step" = one pass of the hot path over a batch of `--tiles` synthetic rectified pairs per GPU.
 `value`  : whole-job Mpix/s with the pairs already resident in HBM (device pointers through
@@ -58,7 +59,47 @@ def parse():
     ap.add_argument("--nan-border", type=float, default=0.0,
                     help="fraction of the tile width turned into no-data strips (0 = the BASELINE workload; > 0 exercises the "
                          "no-data sentinel range, which can widen the right view's slab: DESIGN.md, limits)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the disparity, confidence and rejection mask of the last device-resident step "
+                         "(rank 0's tiles) as DIR/{disp,conf,mask}.npy, float32 of shape (tiles, H, W), and DIR/{disp,conf}_valid.npy "
+                         "(1 where the output is finite, 0 where it is NaN = no match; the value itself is then written as 0); above "
+                         "%d MB in all, the same seeded sample of pixels of each, flattened in (tile, row, column) order" % (DUMP_BYTES // 10 ** 6))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(torch, out_dir, named):
+    """Write the named lists of (H, W) device tensors to out_dir/<name>.npy as float32: whole when they fit DUMP_BYTES together,
+    else each at the same seeded sample of flat indices.  Every file holds finite values only: a floating-point output is written
+    with its non-finite values (NaN marks a pixel without a disparity) set to 0, beside <name>_valid.npy, 1 where it is finite.
+    -> description for the JSON line."""
+    os.makedirs(out_dir, exist_ok=True)
+    first = next(iter(named.values()))
+    nfiles = sum(2 if t[0].is_floating_point() else 1 for t in named.values())
+    total = sum(t.numel() for t in first)
+    n = min(total, (DUMP_BYTES - 4096 * nfiles) // (4 * nfiles))       # 4096: room for the .npy headers
+    idx = None
+    if n < total:
+        rng = np.random.default_rng(0)
+        idx = torch.from_numpy(np.sort(rng.choice(total, size=n, replace=False))).to(first[0].device)
+    names = []
+    for name, tensors in named.items():
+        x = torch.stack(tensors)
+        x = x if idx is None else x.reshape(-1)[idx]
+        out = {name: x.float()}
+        if x.is_floating_point():
+            ok = torch.isfinite(x)
+            out = {name: torch.where(ok, x, torch.zeros_like(x)).float(), name + "_valid": ok.float()}
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy())
+            names.append(k)
+    return {"dir": out_dir, "names": sorted(names), "dtype": "float32",
+            "sampled": None if idx is None else "%d of %d pixels per output, numpy default_rng(0) choice without replacement, sorted" % (n, total)}
 
 
 def config(a, world):
@@ -292,6 +333,9 @@ def run_ours(a, rank, world, local_rank):
     tw1 = time.perf_counter()
     launches = eng.kernel_launches() - l0
     ms = max_over_ranks(e0.elapsed_time(e1))
+    dumped = None
+    if a.dump_outputs and rank == 0:
+        dumped = dump_outputs(torch, a.dump_outputs, {"disp": d_disp, "conf": d_conf, "mask": d_mask})
     # stage durations of the LAST tile of each workspace while the tiles overlap (diagnostic: how much the
     # memory-bound WTA stretches when it shares the SMs with the next tile's aggregation)
     overlapped = {}
@@ -422,6 +466,7 @@ def run_ours(a, rank, world, local_rank):
             "valid_fraction_tile0": valid, "outputs_verified": verified,
             "outputs_verified_how": "all %d tiles of the last timed step (%d in flight) and of the last end-to-end step, bit for bit "
                                     "against a serial re-run of each tile (disparity, confidence, mask)" % (B, nslots),
+            "dumped_outputs": dumped,
         }
     # ---- the other configurations (every rank takes part; rank 0 reports)
     extras = {}

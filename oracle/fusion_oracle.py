@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- numpy restatement of s2p.fusion.merge_n's arithmetic (s2p/fusion.py:16-68).
 
-`merge_ref` runs the REFERENCE's own `average_if_close`, extracted from /root/reference/s2p/fusion.py when that
-tree is present (the module itself cannot be imported here: it needs rasterio), through np.apply_along_axis
+`merge_ref` runs the REFERENCE's own `average_if_close`, extracted from its s2p/fusion.py (S2PB_FUSION_REFERENCE, default:
+the reference tree beside the repository) when that file is present (the module itself cannot be imported here: it needs rasterio), through np.apply_along_axis
 exactly as merge_n does; `merge_port` is the vectorised restatement used where the reference is absent.
 """
 import ast
@@ -10,11 +10,12 @@ import warnings
 
 import numpy as np
 
-REF = "/root/reference/s2p/fusion.py"
+REF = os.environ.get("S2PB_FUSION_REFERENCE") or os.path.join(os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))),
+                                                              "reference", "s2p", "fusion.py")
 
 
 def reference_average_if_close():
-    """-> the reference's function object, or None when /root/reference is absent."""
+    """-> the reference's function object, or None when the reference's fusion.py is absent."""
     if not os.path.exists(REF):
         return None
     tree = ast.parse(open(REF).read())

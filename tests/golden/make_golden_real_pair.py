@@ -6,7 +6,8 @@ rectified_ref.tif, rectified_disp.tif): real Pleiades imagery through the whole 
 * rectified_disp.tif is the reference's disparity for that pair (its rectified_sec.tif is not shipped: it is rebuilt by
   warping img_02.tif with H_sec.txt, and the matcher runs on [-41, 30]).
 
-Only the source crops the two warps need are stored (uint16), with their offsets.  The script checks the fixture with the
+Only the source crops the two warps need are stored (uint16), with their offsets.  The arrays are split over three files
+(real_pair.npz, real_pair_rectified_ref.npz, real_pair_rectified_disp.npz) that each stay under 1 MB; load() merges them.  The script checks the fixture with the
 CPU oracles before writing: the reference resampler compiled in place reproduces rectified_ref.tif, and the reference
 `mgm` on the rebuilt pair reproduces rectified_disp.tif to <= 0.25 px on > 99.5 % of the pixels.
     python tests/golden/make_golden_real_pair.py
@@ -21,6 +22,18 @@ sys.path.insert(0, ROOT)
 REF = "/root/reference/tests/data"
 W, H = 503, 425
 DMIN, DMAX = -41, 30
+
+
+HERE = os.path.dirname(os.path.abspath(__file__))
+RECTIFIED = ("rectified_ref", "rectified_disp")
+
+
+def load():
+    """-> {name: array} of the whole fixture"""
+    z = dict(np.load(os.path.join(HERE, "real_pair.npz")))
+    for name in RECTIFIED:
+        z[name] = np.load(os.path.join(HERE, "real_pair_%s.npz" % name))[name]
+    return z
 
 
 def crop_for(Hm, img, w, h, margin=8):
@@ -67,9 +80,10 @@ def main():
         with Image.open(os.path.join(REF, "input_pair", name)) as im:
             rpcs.append(np.array(im.tag_v2[50844], np.float64))
     assert rpcs[0].size == 92 and rpcs[1].size == 92
-    np.savez_compressed(os.path.join(os.path.dirname(os.path.abspath(__file__)), "real_pair.npz"),
-                        crop1=c1.astype(np.uint16), xy1=np.array(xy1), crop2=c2.astype(np.uint16), xy2=np.array(xy2),
-                        H1=H1, H2=H2, rectified_ref=rect_ref, rectified_disp=rect_disp, rpc1=rpcs[0], rpc2=rpcs[1])
+    np.savez_compressed(os.path.join(HERE, "real_pair.npz"), crop1=c1.astype(np.uint16), xy1=np.array(xy1), crop2=c2.astype(np.uint16),
+                        xy2=np.array(xy2), H1=H1, H2=H2, rpc1=rpcs[0], rpc2=rpcs[1])
+    for name, a in zip(RECTIFIED, (rect_ref, rect_disp)):
+        np.savez_compressed(os.path.join(HERE, "real_pair_%s.npz" % name), **{name: a})
 
 
 if __name__ == "__main__":

@@ -1,9 +1,15 @@
-"""n-view merge (SURVEY.md section 8f rank 1): the numpy restatement against the reference's own
+"""n-view merge (SURVEY.md section 8f rank 1): the numpy restatement against the stored results of the reference's own
 `average_if_close` (CPU), and the CUDA kernel against the restatement (GPU).  Bit-exact."""
+import os
+import sys
+
 import numpy as np
 import pytest
 
 from util import same
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import reference_runs as RR  # noqa: E402
 
 
 def _maps(n, h=37, w=53, seed=0):
@@ -22,11 +28,11 @@ def _maps(n, h=37, w=53, seed=0):
 @pytest.mark.parametrize("n", [2, 3, 5])
 def test_port_matches_reference_function(n):
     from oracle import fusion_oracle as F
-    if F.reference_average_if_close() is None:
-        pytest.skip("/root/reference not present")
     maps, offsets = _maps(n, seed=n)
     for thr in (1, 3):
-        assert same(F.merge_port(maps, offsets, "average_if_close", thr), F.merge_ref(maps, offsets, thr))
+        want = RR.reference_digests("average_if_close/n=%d,threshold=%d" % (n, thr), lambda: {"merged": F.merge_ref(maps, offsets, thr)})
+        bad = RR.mismatches({"merged": F.merge_port(maps, offsets, "average_if_close", thr)}, want)
+        assert not bad, bad
 
 
 @pytest.mark.gpu
@@ -62,22 +68,31 @@ def test_gpu_merge_dropin_files(engine, tmp_path):
     assert same(rio.read_band(out), F.merge_port(maps, offsets, "average_if_close", 3))
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("radius", [2, 3, 5])
-def test_gpu_mask_erosion_matches_reference(engine, oracle, radius, tmp_path):
-    """masking.erosion = `morsi diskR erosion` (c/morsi.c compiled in place as oracle/_ref/libmorsi_ref.so)."""
-    if not oracle.have_ref_morsi():
-        pytest.skip("oracle/_ref/libmorsi_ref.so not built")
+EROSION_RADII = [2, 3, 5]
+
+
+def erosion_reference(oracle, radius):
+    """-> (mask, stored digests of the reference's erosion of it)"""
     rng = np.random.default_rng(radius)
     m = (rng.random((61, 83)) > 0.15).astype(np.uint8)
-    want = oracle.ref_disk_erosion(m.astype(np.float32), radius).astype(np.uint8)
-    assert np.array_equal(engine.erode_mask(m, radius), want)
+    want = RR.reference_digests("disk_erosion/%d" % radius,
+                                lambda: {"mask": oracle.ref_disk_erosion(m.astype(np.float32), radius).astype(np.uint8)})
+    return m, want
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("radius", EROSION_RADII)
+def test_gpu_mask_erosion_matches_reference(engine, oracle, radius, tmp_path):
+    """masking.erosion = `morsi diskR erosion` (c/morsi.c compiled in place as oracle/_ref/libmorsi_ref.so; its results are
+    stored by tests/golden/reference_runs.py)."""
+    m, want = erosion_reference(oracle, radius)
+    assert not RR.mismatches({"mask": engine.erode_mask(m, radius)}, want)
     if radius == 2:       # file-level drop-in (s2p/masking.py:87-97)
         from s2p_b200 import masking, rasterio_compat as rio
         p = str(tmp_path / "rectified_mask.png")
         rio.write_mask_png(p, m)
         masking.erosion(p, p, 2)
-        assert np.array_equal(rio.read_band(p).astype(np.uint8), want)
+        assert not RR.mismatches({"mask": rio.read_band(p).astype(np.uint8)}, want)
         rio.write_mask_png(p, m)
         masking.erosion(p, p, 1)                      # below 2: untouched, as in the reference
         assert np.array_equal(rio.read_band(p).astype(np.uint8), m)

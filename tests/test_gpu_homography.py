@@ -4,10 +4,17 @@ The checker is oracle/_ref/homography_ref: the UNMODIFIED LibHomography / LibIma
 compiled in place behind oracle/homography_harness.cpp.  The reference is float32 + SSE and is built with
 -O3 -march=native, so its own output depends on FMA contraction: two builds of the same sources
 (oracle/_ref/homography_ref vs homography_ref_nofma) differ by up to 6e-5 of the dynamic range on these inputs.
-The tolerance below is set from that spread: |ours - reference| <= 1e-4 * max|src| on every pixel, and the
-NaN (outside-the-source) masks are identical except for pixels lying exactly on the source boundary."""
+The tolerance below is set from that spread: |ours - reference| <= 1e-4 * max|src|, and the NaN (outside-the-source)
+masks are identical except for pixels lying exactly on the source boundary.  The reference's outputs are stored by
+tests/golden/reference_runs.py: the NaN mask in full, the values on a seeded sample of 2048 pixels."""
+import os
+import sys
+
 import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import reference_runs as RR  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 REL_TOL = 1e-4
@@ -38,40 +45,46 @@ CASES = {
 }
 
 
-@pytest.mark.parametrize("name", sorted(CASES))
-def test_warp_matches_reference(engine, oracle, name):
-    if not oracle.have_ref_homography():
-        pytest.skip("oracle/_ref/homography_ref not built")
-    src = _src()
-    H = CASES[name]
-    ow, oh = 256, 200
-    ref = oracle.run_ref_homography(src, H, ow, oh)
-    got = engine.homography(src, H, ow, oh)
-    assert got.shape == ref.shape == (oh, ow)
-    nan_diff = int((np.isnan(ref) != np.isnan(got)).sum())
-    assert nan_diff <= max(2, ref.size // 5000), "%d NaN-mask mismatches" % nan_diff
-    both = np.isfinite(ref) & np.isfinite(got)
-    assert both.any()
-    err = np.abs(ref[both] - got[both]).max()
+def warp_reference(oracle, name):
+    """-> the stored reference resampler's output (reference_runs.Sample) for CASES[name] on _src(), 256 x 200"""
+    return RR.reference_samples("warp/" + name, lambda: {"out": oracle.run_ref_homography(_src(), CASES[name], 256, 200)})["out"]
+
+
+def dropin_reference(oracle):
+    """-> (source, homography, stored reference output 200 x 150) of the file drop-in test"""
+    src, H = _src(260, 340, seed=3, nan=False), _rot(0.12, 1.0, 20, -15)
+    return src, H, RR.reference_samples("warp_dropin", lambda: {"out": oracle.run_ref_homography(src, H, 200, 150)})["out"]
+
+
+def _assert_close(got, want, src, max_nan_diff):
+    assert got.shape == want.shape
+    nan_diff = int((want.isnan != np.isnan(got)).sum())
+    assert nan_diff <= max_nan_diff, "%d NaN-mask mismatches" % nan_diff
+    assert (~want.isnan & np.isfinite(got)).any()
+    g = want.at(got)
+    both = np.isfinite(want.val) & np.isfinite(g)
+    err = np.abs(want.val[both] - g[both]).max()
     assert err <= REL_TOL * np.nanmax(np.abs(src)), "max abs error %g" % err
 
 
+@pytest.mark.parametrize("name", sorted(CASES))
+def test_warp_matches_reference(engine, oracle, name):
+    want = warp_reference(oracle, name)
+    got = engine.homography(_src(), CASES[name], 256, 200)
+    assert got.shape == (200, 256)
+    _assert_close(got, want, _src(), max(2, got.size // 5000))
+
+
 def test_dropin_file_contract(engine, oracle, tmp_path):
-    if not oracle.have_ref_homography():
-        pytest.skip("oracle/_ref/homography_ref not built")
     import subprocess
     from s2p_b200 import common, rasterio_compat as rio
-    src = _src(260, 340, seed=3, nan=False)
+    src, H, want = dropin_reference(oracle)
     im, out = str(tmp_path / "im.tif"), str(tmp_path / "rect.tif")
     rio.write_float_tiff(im, src)
-    H = _rot(0.12, 1.0, 20, -15)
     assert common.image_apply_homography(out, im, H, 200, 150) is None
     got = rio.read_band(out)
-    ref = oracle.run_ref_homography(src, H, 200, 150)
     assert got.shape == (150, 200)
-    assert int((np.isnan(ref) != np.isnan(got)).sum()) <= 2
-    both = np.isfinite(ref) & np.isfinite(got)
-    assert np.abs(ref[both] - got[both]).max() <= REL_TOL * np.abs(src).max()
+    _assert_close(got, want, src, 2)
     with pytest.raises(subprocess.CalledProcessError):      # the binary exits with "empty roi"
         common.image_apply_homography(out, im, _rot(0, 1.0, 5000, 5000), 50, 50)
 
@@ -94,8 +107,8 @@ def test_dropin_warps_every_band(engine, oracle, tmp_path):
 
 
 def _real_pair():
-    import os
-    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "real_pair.npz"))
+    import make_golden_real_pair
+    z = make_golden_real_pair.load()
     comp = lambda Hm, xy: np.asarray(Hm, np.float64) @ np.array([[1, 0, xy[0]], [0, 1, xy[1]], [0, 0, 1.0]])
     return z, comp(z["H1"], z["xy1"]), comp(z["H2"], z["xy2"])
 

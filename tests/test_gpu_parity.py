@@ -2,11 +2,17 @@
 seeded inputs.  Bit-exact for the integer WTA index, confidence, mask and -- because the
 device arithmetic follows the reference's float32 operation order -- for the sub-pixel map too
 (the contract only asks +-0.25 px; both are asserted, the tolerance stated here)."""
+import os
+import sys
+
 import numpy as np
 import pytest
 
 from s2p_b200.synth import make_pair
 from util import nmismatch, same
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import reference_runs as RR  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 SUBPIX_TOL = 0.25  # px, BASELINE.json north_star
@@ -260,21 +266,32 @@ def test_batch_page_locked_buffers_match_staged(engine):
         eng.mgm_batch(refs, secs, -12, 9, p, out=(outs[0][:2], outs[1], outs[2]))
 
 
-@pytest.mark.parametrize("shape,dmin,dmax,nanb,seed", [((56, 88), -10, 9, 0.07, 106), ((90, 203), -24, 23, 0.05, 7), ((64, 333), -9, 40, 0.1, 8)])
+NODATA_CASES = [((56, 88), -10, 9, 0.07, 106), ((90, 203), -24, 23, 0.05, 7), ((64, 333), -9, 40, 0.1, 8)]
+
+
+def nodata_reference(oracle, shape, dmin, dmax, nanb, seed):
+    """-> (ref, sec, stored digests of the reference binary's disp / conf / dispR on them)"""
+    h, w = shape
+    ref, sec, _ = make_pair(h, w, dmin, dmax, seed=seed, nan_border=nanb)
+
+    def run():
+        r = oracle.run_ref(ref, sec, dmin, dmax, oracle.mgm_params(), threads=1)
+        return {k: r[k] for k in ("disp", "conf", "dispR")}
+    return ref, sec, RR.reference_digests("nodata/%dx%d,seed=%d" % (h, w, seed), run)
+
+
+@pytest.mark.parametrize("shape,dmin,dmax,nanb,seed", NODATA_CASES)
 def test_nodata_matches_reference_binary(engine, oracle, shape, dmin, dmax, nanb, seed):
     """No-data in BOTH images: the reference's DCT round trip of the matched image leaves rounding noise on the zeroed
     pixels (mgm_costvolume.cc:23-60), which the census transform then compares.  The engine reproduces the round trip with
-    the same tables and summation order, so it equals the unmodified reference binary bit for bit on such tiles too."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/mgm not built")
+    the same tables and summation order, so it equals the unmodified reference binary bit for bit on such tiles too
+    (its outputs are stored by tests/golden/reference_runs.py)."""
     from s2p_b200.engine import default_params
-    h, w = shape
-    ref, sec, _ = make_pair(h, w, dmin, dmax, seed=seed, nan_border=nanb)
+    ref, sec, want = nodata_reference(oracle, shape, dmin, dmax, nanb, seed)
     assert np.isnan(ref).any() and np.isnan(sec).any()
-    r = oracle.run_ref(ref, sec, dmin, dmax, oracle.mgm_params(), threads=1)
     out = engine.mgm(ref, sec, dmin, dmax, default_params("mgm"), want_right=True)
-    assert same(out["disp"], r["disp"]), "%d px differ from the reference binary" % nmismatch(out["disp"], r["disp"])
-    assert same(out["conf"], r["conf"]) and same(out["disp_right"], r["dispR"])
+    bad = RR.mismatches(dict(disp=out["disp"], conf=out["conf"], dispR=out["disp_right"]), want)
+    assert not bad, "differs from the reference binary: " + "; ".join(bad)
 
 
 def test_exact_zero_pixels_without_nodata(engine, oracle):
@@ -331,17 +348,26 @@ def test_eight_tiles_in_flight_equal_serial(engine):
             assert same(conf[k], one["conf"]) and np.array_equal(mask[k], one["mask"])
 
 
-def test_rejection_mask_matches_reference_programs(engine, oracle):
-    """the mask kernel against the reference's own plambda / backflow / plambda chain (oracle/_ref, c/*.c compiled in place)"""
-    if not oracle.have_ref_mask():
-        pytest.skip("oracle/_ref/backflow not built")
+def rejection_mask_reference(oracle):
+    """-> [(disp, ref, sec, stored digests of the reference programs' mask)] for two tiles"""
     rng = np.random.default_rng(4)
+    out = []
     for seed, (h, w, dmin, dmax) in enumerate([(70, 110, -12, 12), (45, 200, -30, 8)]):
         ref, sec, gt = make_pair(h, w, dmin, dmax, seed=50 + seed, nan_border=0.06)
         d = gt + rng.uniform(-0.7, 0.7, gt.shape).astype(np.float32)
         d[rng.random(d.shape) < 0.1] = np.nan
         d[:, :3] -= 7.3
-        assert np.array_equal(engine.rejection_mask(d, ref, sec), oracle.ref_rejection_mask(d, ref, sec))
+        want = RR.reference_digests("rejection_mask_gpu/%d" % seed, lambda: {"mask": oracle.ref_rejection_mask(d, ref, sec)})
+        out.append((d, ref, sec, want))
+    return out
+
+
+def test_rejection_mask_matches_reference_programs(engine, oracle):
+    """the mask kernel against the reference's own plambda / backflow / plambda chain (oracle/_ref, c/*.c compiled in place; its
+    results are stored by tests/golden/reference_runs.py)"""
+    for d, ref, sec, want in rejection_mask_reference(oracle):
+        bad = RR.mismatches({"mask": engine.rejection_mask(d, ref, sec)}, want)
+        assert not bad, bad
 
 
 def test_mgm_multi_level_hull_wider_than_512_labels(engine, oracle):

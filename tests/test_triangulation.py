@@ -1,9 +1,16 @@
 """Triangulation (SURVEY.md section 8f rank 2): the CUDA kernel against the reference's own disp_to_lonlatalt
 (c/disp_to_h.c + c/rpc.c compiled in place as oracle/_ref/libdisp_to_h_ref.so).  float64 iterative geometry built
 -O3 -march=native on the reference side: tolerance 1e-9 degree (~0.1 mm) on lon/lat, 1e-6 m on the altitude,
-1e-4 px on the reprojection error, identical NaN pattern."""
+1e-4 px on the reprojection error, identical NaN pattern.  The reference library's outputs are stored by
+tests/golden/reference_runs.py: the NaN patterns in full, the values on a seeded sample of pixels."""
+import os
+import sys
+
 import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import reference_runs as RR  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -49,11 +56,18 @@ def _geometry():
     return H1, H2, (4180.0, 4330.0, 3280.0, 3390.0)
 
 
-@pytest.mark.parametrize("with_direct", [False, True])
-def test_matches_reference_library(engine, oracle, with_direct):
-    if not oracle.have_ref_triangulation():
-        pytest.skip("oracle/_ref/libdisp_to_h_ref.so not built")
-    from s2p_b200.triangulation import disp_to_lonlatalt
+def _assert_matches(got, gerr, want, min_valid):
+    w, werr = want["lonlatalt"], want["err"]
+    assert np.array_equal(w.isnan, np.isnan(got)) and np.array_equal(werr.isnan, np.isnan(gerr))
+    assert (~w.isnan[..., 0]).mean() > min_valid
+    wv, gv, we, ge = w.val, w.at(got), werr.val, werr.at(gerr)
+    ok = np.isfinite(wv[:, 0])
+    assert np.abs(wv[ok][:, :2] - gv[ok][:, :2]).max() < 1e-9
+    assert np.abs(wv[ok][:, 2] - gv[ok][:, 2]).max() < 1e-6
+    assert np.abs(we[ok] - ge[ok]).max() < 1e-4
+
+
+def synthetic_inputs(with_direct):
     rng = np.random.default_rng(5)
     h, w = 60, 90
     rpc1, rpc2 = _rpc(1, with_direct), _rpc(2, with_direct)
@@ -61,25 +75,14 @@ def test_matches_reference_library(engine, oracle, with_direct):
     mask = (rng.random((h, w)) > 0.2).astype(np.float32)
     H1, H2, bbx = _geometry()
     mo = (rng.random((int(bbx[3] - bbx[2]) + 1, int(bbx[1] - bbx[0]) + 1)) > 0.1).astype(np.float32)
-    want, werr = oracle.ref_disp_to_lonlatalt(disp, mask, mo, H1, H2, rpc1, rpc2, bbx)
-    got, gerr = disp_to_lonlatalt(disp, mask, mo, H1, H2, rpc1, rpc2, bbx, engine=engine)
-    assert np.array_equal(np.isnan(want), np.isnan(got)) and np.array_equal(np.isnan(werr), np.isnan(gerr))
-    ok = np.isfinite(want[..., 0])
-    assert ok.mean() > 0.3
-    assert np.abs(want[ok][:, :2] - got[ok][:, :2]).max() < 1e-9
-    assert np.abs(want[ok][:, 2] - got[ok][:, 2]).max() < 1e-6
-    assert np.abs(werr[ok] - gerr[ok]).max() < 1e-4
+    return disp, mask, mo, H1, H2, rpc1, rpc2, bbx
 
 
-def test_real_rpc_real_disparity(engine, oracle):
-    """Real cameras: the RPCs of the reference's Pleiades fixture (tests/data/input_pair/img_0{1,2}.tif, RPCCoefficientTag,
-    ground->image polynomials only, so every localisation runs the Newton iteration of c/rpc.c:378-411), its rectifying
-    homographies and its shipped disparity map (tests/golden/real_pair.npz), against the reference library."""
-    import os
-    if not oracle.have_ref_triangulation():
-        pytest.skip("oracle/_ref/libdisp_to_h_ref.so not built")
-    from s2p_b200.triangulation import disp_to_lonlatalt, rpc_from_geotiff_tag
-    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "real_pair.npz"))
+def real_inputs():
+    """Real cameras: the RPCs of the reference's Pleiades fixture, its rectifying homographies and its shipped disparity map"""
+    import make_golden_real_pair
+    from s2p_b200.triangulation import rpc_from_geotiff_tag
+    z = make_golden_real_pair.load()
     rpc1, rpc2 = rpc_from_geotiff_tag(z["rpc1"]), rpc_from_geotiff_tag(z["rpc2"])
     disp = z["rectified_disp"][100:260, 120:360].copy()
     # the rectified crop starts at (120, 100): move the origin into the homographies
@@ -90,13 +93,33 @@ def test_real_rpc_real_disparity(engine, oracle):
     bbx = (0.0, 1023.0, 0.0, 1023.0)
     mo = np.ones((1024, 1024), np.float32)
     mo[300:340, 500:560] = 0          # a hole in the image-domain mask
-    want, werr = oracle.ref_disp_to_lonlatalt(disp, mask, mo, H1, H2, rpc1, rpc2, bbx)
-    got, gerr = disp_to_lonlatalt(disp, mask, mo, H1, H2, rpc1, rpc2, bbx, engine=engine)
-    assert np.array_equal(np.isnan(want), np.isnan(got)) and np.array_equal(np.isnan(werr), np.isnan(gerr))
-    ok = np.isfinite(want[..., 0])
-    assert ok.mean() > 0.5
-    assert np.abs(want[ok][:, :2] - got[ok][:, :2]).max() < 1e-9
-    assert np.abs(want[ok][:, 2] - got[ok][:, 2]).max() < 1e-6
-    assert np.abs(werr[ok] - gerr[ok]).max() < 1e-4
+    return (disp, mask, mo, H1, H2, rpc1, rpc2, bbx), z
+
+
+def triangulation_reference(oracle, key, args):
+    def run():
+        out, err = oracle.ref_disp_to_lonlatalt(*args)
+        return {"lonlatalt": out, "err": err}
+    return RR.reference_samples("disp_to_lonlatalt/" + key, run)
+
+
+@pytest.mark.parametrize("with_direct", [False, True])
+def test_matches_reference_library(engine, oracle, with_direct):
+    from s2p_b200.triangulation import disp_to_lonlatalt
+    args = synthetic_inputs(with_direct)
+    want = triangulation_reference(oracle, "synthetic_direct=%d" % with_direct, args)
+    got, gerr = disp_to_lonlatalt(*args, engine=engine)
+    _assert_matches(got, gerr, want, 0.3)
+
+
+def test_real_rpc_real_disparity(engine, oracle):
+    """Real cameras: the RPCs of the reference's Pleiades fixture (tests/data/input_pair/img_0{1,2}.tif, RPCCoefficientTag,
+    ground->image polynomials only, so every localisation runs the Newton iteration of c/rpc.c:378-411), its rectifying
+    homographies and its shipped disparity map (tests/golden/real_pair*.npz), against the reference library."""
+    from s2p_b200.triangulation import disp_to_lonlatalt
+    args, z = real_inputs()
+    want = triangulation_reference(oracle, "real", args)
+    got, gerr = disp_to_lonlatalt(*args, engine=engine)
+    _assert_matches(got, gerr, want, 0.5)
     # plausibility: the fixture is over the Reunion island area of the RPC offsets, altitudes within the RPC's height range
     assert abs(np.nanmedian(got[..., 0]) - z["rpc1"][5]) < 0.2 and abs(np.nanmedian(got[..., 1]) - z["rpc1"][4]) < 0.2
